@@ -3,9 +3,11 @@
 
 Contract (see the task statement): `python bench.py --gpus N --steps K --warmup W` (torchrun for N>1) prints ONE JSON
 line on rank 0.  One "step" = one pass of the hot path over one batch of `--windows` independent tracking windows per GPU
-(BASELINE.json configs[1] replicated; configs[3] is 32 windows/GPU x 8 GPUs), i.e. weak scaling.  Every timed region runs its
-K-step block back to back until --min-seconds have passed (CUDA events around every block, median block reported, max over
-ranks), so the clocks sampled during the region mean something.
+(BASELINE.json configs[1] replicated; configs[3] is 32 windows/GPU x 8 GPUs), i.e. weak scaling.  Every timed region runs
+exactly K steps between CUDA events (max over ranks).  --min-seconds S repeats that K-step block back to back until S seconds have
+passed and reports the median block, so that the clocks sampled during the region mean something.  --dump-outputs DIR writes the
+poses the timed paths returned in their last step (value: poses.npy, e2e: e2e_poses.npy, [windows, frames, 4, 4] float32); the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
   value     windows/s, whole job, inputs (keyframe maps, correspondences, poses, tables) already resident in HBM: per step
             ONE new frame per window is stored into the keyframe cache (k_frame_cache_store: its quarter-resolution maps are
@@ -52,8 +54,9 @@ def parse():
     ap.add_argument("--scenes", type=int, default=4, help="distinct rendered scenes per GPU; windows cycle through them with their own pose noise and their own copy of the frame maps")
     ap.add_argument("--cpu-windows", type=int, default=0, help="cpu_baseline sample size (0 = 2 per core)")
     ap.add_argument("--ref-windows", type=int, default=8, help="windows per step for --impl reference")
-    ap.add_argument("--min-seconds", type=float, default=1.0, help="each timed region repeats its K-step block until it has run this long")
+    ap.add_argument("--min-seconds", type=float, default=0.0, help="repeat each timed region's K-step block until it has run this long (default: K steps once)")
     ap.add_argument("--skip-cfg3", action="store_true", help="leave out the BASELINE configs[2] block (30-keyframe pool)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the poses of the timed paths' last step to DIR/*.npy (--impl ours)")
     return ap.parse_args()
 
 
@@ -582,7 +585,13 @@ def main():
         for t in (t_val, t_e2e, t_rb, t_sync):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         from bundletrack_b200.sharding import gather_poses   # NCCL only gathers the results (windows are sharded per rank)
-        gather_poses(poses, args.windows * world, [N] * (args.windows * world), rank, world, device=dev)
+        poses = gather_poses(poses, args.windows * world, [N] * (args.windows * world), rank, world, device=dev)
+        if args.dump_outputs:
+            out_poses = gather_poses(out_poses, args.windows * world, [N] * (args.windows * world), rank, world, device=dev)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "poses.npy"), np.stack(poses).astype(np.float32))
+        np.save(os.path.join(args.dump_outputs, "e2e_poses.npy"), np.stack(out_poses).astype(np.float32))
     ms_step = float(t_val.item())
     value = world * args.windows / (ms_step * 1e-3)
     e2e_val = world * args.windows / (float(t_e2e.item()) * 1e-3)

@@ -267,19 +267,21 @@ def test_ransac_matches_reference_golden(cuda_device):
 
 
 def test_ransac_matches_reference_live(cuda_device):
-    """The reference's own kernels run live on this GPU (oracle/_ref): n = 8 ... 3000 points, and the 45 pairs of a 10-keyframe
-    window at cfg2 sizes in one call.  Identical inlier sets are the rule; a pair may differ only as _ransac_vs_reference allows."""
-    import oracle
-    if not os.path.exists(os.path.join(os.path.dirname(oracle.__file__), "_ref", "libbt_ref.so")):
-        pytest.skip("oracle/_ref not built")
+    """The reference's own ransacMultiPairGPU (its inlier sets recorded on a B200 in tests/golden/ref_matcher_runs.npz, made by
+    scripts/make_golden_reference_runs.py): n = 8 ... 3000 points, and the 45 pairs of a 10-keyframe window at cfg2 sizes in one
+    call.  Identical inlier sets are the rule; a pair may differ only as _ransac_vs_reference allows."""
+    g = np.load(os.path.join(GOLD, "ref_matcher_runs.npz"))
+    def ref_ids(key, n):
+        return np.flatnonzero(np.unpackbits(g[key], count=n)).astype(np.int32)
     verdicts = []
     for n, thresh in ((8, 0.005), (60, 0.005), (300, 0.01), (1000, 0.005), (3000, 0.005)):
         cases = [_ransac_case(7000 + 10 * n + k, n, inlier_frac=0.5 + 0.1 * k) for k in range(3)]
-        ref, _ = oracle.ref_ransac_pairs([c[0] for c in cases], [c[1] for c in cases], 2000, thresh)
+        ref = [ref_ids(f"ransac_n{n}_{k}", n) for k in range(3)]
         verdicts += _ransac_reference_check(cuda_device, [c[0] for c in cases], [c[1] for c in cases], ref, thresh, f"n{n}")
     rng = np.random.default_rng(5)
     cases = [_ransac_case(8000 + p, int(rng.integers(300, 1600)), inlier_frac=float(rng.uniform(0.3, 0.9))) for p in range(45)]
-    ref, _ = oracle.ref_ransac_pairs([c[0] for c in cases], [c[1] for c in cases], 2000, 0.005)
+    assert np.array_equal([len(c[0]) for c in cases], g["ransac_cfg2_n"])      # the inputs the reference was run on
+    ref = [ref_ids(f"ransac_cfg2_{p}", len(c[0])) for p, c in enumerate(cases)]
     verdicts += _ransac_reference_check(cuda_device, [c[0] for c in cases], [c[1] for c in cases], ref, 0.005, "cfg2")
     print("RANSAC vs reference:", {v: verdicts.count(v) for v in sorted(set(verdicts))})
     assert verdicts.count("identical") >= int(0.6 * len(verdicts)), verdicts
@@ -363,35 +365,38 @@ def test_fused_pipeline_matches_oracle_and_feeds_solver(cuda_device):
     depth = [f["depth"] for f in devf]; normal = [f["normal"] for f in devf]
     out = opt.optimizeWindows([SolveWindow(ent, w.H, w.W, depth, normal, w.poses_init, w.K)])[0]
     # same RANSAC winner on both sides (the device's own entries handed to the oracle solver): north_star's 1e-4 rad / 1e-4 m
-    if os.path.exists(os.path.join(os.path.dirname(oracle.__file__), "_ref", "libbt_ref.so")):
-        ref_same, pairs, _, _ = oracle.ref_optimize_frames([d.data_ptr() for d in depth], [n.data_ptr() for n in normal], w.H, w.W, w.K, ent, w.poses_init)
-        out_same = opt.optimizeWindows([SolveWindow(ent, w.H, w.W, depth, normal, w.poses_init, w.K, dense_pairs=pairs)])[0]
-        r, t = synth.pose_errors(out_same, ref_same)
-        # yardsticks on this very window: the reference against itself (float atomics: its sums change from run to run) and the IEEE
-        # restatement of the same arithmetic (oracle A, same pair directions) against the reference.  On a window whose hard dense gates
-        # amplify rounding (tests/test_solver_gpu.py::test_gate_sensitive_window) no implementation can be closer to the reference than
-        # those two are; on all others the plain 1e-4 applies.
-        ref_again = oracle.ref_optimize_frames([d.data_ptr() for d in depth], [n.data_ptr() for n in normal], w.H, w.W, w.K, ent, w.poses_init)[0]
-        a_same = oracle.solve_window(w.depth, w.normal, w.K, ent, w.poses_init, pairs=pairs)
-        yard = max(max(synth.pose_errors(ref_again, ref_same)), max(synth.pose_errors(a_same, ref_same)))
-        print(f"fused chain -> solver vs the reference's kernels on the same entries: rot {r:.2e} rad trans {t:.2e} m "
-              f"(reference run-to-run {max(synth.pose_errors(ref_again, ref_same)):.2e}, oracle A vs reference {max(synth.pose_errors(a_same, ref_same)):.2e})")
-        a64_same = oracle.solve_window(w.depth, w.normal, w.K, ent, w.poses_init, pairs=pairs, precision="f64")
-        print(f"   pair directions {np.asarray(pairs).tolist()}; oracle float vs double {max(synth.pose_errors(a_same, a64_same)):.2e}; library vs oracle float {max(synth.pose_errors(out_same, a_same)):.2e}, vs oracle double {max(synth.pose_errors(out_same, a64_same)):.2e}")
-        if max(r, t) > max(1e-4, 1.25 * yard):
-            # ONE source pixel of pair (3,0) of this window sits on the 2 cm distance gate: depending on rounding-level differences of the
-            # poses of the earlier iterations (e.g. the order in which the pairs' sums are added - the reference's pair list changes with
-            # its allocation addresses) it is gated in or out, the pair's count is 771 or 772, and the result moves by 1.5e-4
-            # (scripts/dev_pair_order.py: same pair SET in five orders -> 3e-6 or 1.5e-4, in round 1's solver as well).  When the
-            # tolerance is missed it must be exactly that: a gate count that differs from the oracle's, and poses still within a few 1e-4.
-            opt.enable_debug(True)
-            opt.optimizeWindows([SolveWindow(ent, w.H, w.W, depth, normal, w.poses_init, w.K, dense_pairs=pairs)])
-            cnt = opt.debug_counts(0, len(pairs)).astype(np.int64)
-            opt.enable_debug(False)
-            before_last = oracle.solve_window(w.depth, w.normal, w.K, ent, w.poses_init, pairs=pairs, params=oracle.default_params(num_iter_outer=6))
-            _, _, nf = oracle.dense_system(w.depth, w.normal, w.K, before_last, pairs=pairs)
-            print(f"   gate counts of the last iteration: library {cnt.tolist()}, oracle {nf.tolist()}")
-            assert (cnt != nf).any() and np.abs(cnt - nf).sum() <= 4 and max(r, t) <= 5e-4, (r, t, yard, cnt, nf)
+    # the reference's own kernels on an EntryJ list of this chain (recorded on a B200 with its pair directions and a second run of the
+    # same call, tests/golden/ref_matcher_runs.npz): the library solves that very list
+    g = np.load(os.path.join(GOLD, "ref_matcher_runs.npz"))
+    assert np.allclose(w.poses_init, g["fused_init"], rtol=0, atol=1e-6)
+    ent_ref = g["fused_ent"].view(synth.ENTRYJ_DTYPE).reshape(-1)
+    ref_same, pairs, ref_again = g["fused_poses"], g["fused_pairs"], g["fused_poses_again"]
+    out_same = opt.optimizeWindows([SolveWindow(ent_ref, w.H, w.W, depth, normal, w.poses_init, w.K, dense_pairs=pairs)])[0]
+    r, t = synth.pose_errors(out_same, ref_same)
+    # yardsticks on this very window: the reference against itself (float atomics: its sums change from run to run) and the IEEE
+    # restatement of the same arithmetic (oracle A, same pair directions) against the reference.  On a window whose hard dense gates
+    # amplify rounding (tests/test_solver_gpu.py::test_gate_sensitive_window) no implementation can be closer to the reference than
+    # those two are; on all others the plain 1e-4 applies.
+    a_same = oracle.solve_window(w.depth, w.normal, w.K, ent_ref, w.poses_init, pairs=pairs)
+    yard = max(max(synth.pose_errors(ref_again, ref_same)), max(synth.pose_errors(a_same, ref_same)))
+    print(f"fused chain -> solver vs the reference's kernels on the same entries: rot {r:.2e} rad trans {t:.2e} m "
+          f"(reference run-to-run {max(synth.pose_errors(ref_again, ref_same)):.2e}, oracle A vs reference {max(synth.pose_errors(a_same, ref_same)):.2e})")
+    a64_same = oracle.solve_window(w.depth, w.normal, w.K, ent_ref, w.poses_init, pairs=pairs, precision="f64")
+    print(f"   pair directions {np.asarray(pairs).tolist()}; oracle float vs double {max(synth.pose_errors(a_same, a64_same)):.2e}; library vs oracle float {max(synth.pose_errors(out_same, a_same)):.2e}, vs oracle double {max(synth.pose_errors(out_same, a64_same)):.2e}")
+    if max(r, t) > max(1e-4, 1.25 * yard):
+        # ONE source pixel of pair (3,0) of this window sits on the 2 cm distance gate: depending on rounding-level differences of the
+        # poses of the earlier iterations (e.g. the order in which the pairs' sums are added - the reference's pair list changes with
+        # its allocation addresses) it is gated in or out, the pair's count is 771 or 772, and the result moves by 1.5e-4
+        # (scripts/dev_pair_order.py: same pair SET in five orders -> 3e-6 or 1.5e-4, in round 1's solver as well).  When the
+        # tolerance is missed it must be exactly that: a gate count that differs from the oracle's, and poses still within a few 1e-4.
+        opt.enable_debug(True)
+        opt.optimizeWindows([SolveWindow(ent_ref, w.H, w.W, depth, normal, w.poses_init, w.K, dense_pairs=pairs)])
+        cnt = opt.debug_counts(0, len(pairs)).astype(np.int64)
+        opt.enable_debug(False)
+        before_last = oracle.solve_window(w.depth, w.normal, w.K, ent_ref, w.poses_init, pairs=pairs, params=oracle.default_params(num_iter_outer=6))
+        _, _, nf = oracle.dense_system(w.depth, w.normal, w.K, before_last, pairs=pairs)
+        print(f"   gate counts of the last iteration: library {cnt.tolist()}, oracle {nf.tolist()}")
+        assert (cnt != nf).any() and np.abs(cnt - nf).sum() <= 4 and max(r, t) <= 5e-4, (r, t, yard, cnt, nf)
     ref_same = oracle.solve_window(w.depth, w.normal, w.K, ent, w.poses_init)
     r, t = synth.pose_errors(out, ref_same)
     assert r <= 2e-4 and t <= 1e-4, (r, t)      # Oracle A on this window sits 1.5e-4 from the CUDA path (a gate-sensitive one, see tests/test_solver_gpu.py)

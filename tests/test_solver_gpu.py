@@ -1,5 +1,6 @@
 """GPU parity tests of the CUDA solver (through the C-ABI) against Oracle A (CPU restatement), the committed golden
-vectors of the reference's kernels, and — when oracle/_ref is present — the reference's own kernels run live.
+vectors of the reference's kernels, and the reference's own kernels' poses on further seeded windows, recorded on a B200
+(tests/golden/ref_solver_runs.npz, scripts/make_golden_reference_runs.py).
 Tolerance everywhere: north_star's 1e-4 rad / 1e-4 m after the same 7x5 iterations."""
 import glob
 import os
@@ -13,6 +14,10 @@ from bundletrack_b200 import synth
 pytestmark = pytest.mark.gpu
 TOL = 1e-4
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def _ref_runs():
+    return np.load(os.path.join(GOLD, "ref_solver_runs.npz"))
 
 
 def _upload(w, dev):
@@ -262,13 +267,13 @@ def test_matches_reference_kernels_golden(cuda_device, path):
 
 
 def test_matches_reference_kernels_live(opt, cuda_device):
-    """Oracle B live: the reference's own kernels on this GPU, same inputs, its pair directions fed to both."""
-    if not os.path.exists(os.path.join(os.path.dirname(oracle.__file__), "_ref", "libbt_ref.so")):
-        pytest.skip("oracle/_ref not built")
+    """Oracle B: the reference's own kernels on the same inputs (their poses and pair directions recorded on a B200), its pair
+    directions fed to both."""
+    g = _ref_runs()
     for seed, N, C in ((0, 10, 2000), (40, 6, 1200)):
         w = synth.make_window(seed, n_frames=N, n_corr=C)
-        depth, normal = _upload(w, cuda_device)
-        ref, pairs, _, _ = oracle.ref_optimize_frames([d.data_ptr() for d in depth], [n.data_ptr() for n in normal], w.H, w.W, w.K, w.corr, w.poses_init)
+        assert np.allclose(w.poses_init, g[f"w{seed}_init"], rtol=0, atol=1e-6)      # the inputs the reference was run on
+        ref, pairs = g[f"w{seed}_poses"], g[f"w{seed}_pairs"]
         out = _solve(opt, w, cuda_device, dense_pairs=pairs)
         r, t = synth.pose_errors(out, ref)
         assert r <= TOL and t <= TOL, (seed, r, t)
@@ -415,7 +420,7 @@ def test_prepared_argument_blocks_equal_the_convenience_calls(cuda_device):
 def test_cfg3_whole_pool_window_n30(cuda_device):
     """BASELINE configs[2] with max_BA_frames overridden to the whole 30-keyframe pool: 435 dense pairs, 3000 correspondences,
     YCBInEOAT-style occlusion; a 174 x 174 system (the groups' moment sums stay in global memory: the tail's shared memory would not
-    hold them).  Against Oracle A and, when oracle/_ref is present, the reference's own kernels run live."""
+    hold them).  Against Oracle A and the reference's own kernels (their poses and pair directions recorded on a B200)."""
     from bundletrack_b200.optimizer import OptimizerGpu, SolveWindow
     w = synth.make_window(63, n_frames=30, n_corr=3000, occlusion=True)
     depth, normal = _upload(w, cuda_device)
@@ -427,44 +432,46 @@ def test_cfg3_whole_pool_window_n30(cuda_device):
     assert synth.pose_errors(out, w.poses_gt)[0] < synth.pose_errors(w.poses_init, w.poses_gt)[0]
     again = o.optimizeWindows([SolveWindow(w.corr, w.H, w.W, depth, normal, w.poses_init, w.K)] * 2)
     assert np.array_equal(again[0], again[1])
-    if os.path.exists(os.path.join(os.path.dirname(oracle.__file__), "_ref", "libbt_ref.so")):
-        ref_b, pairs, _, _ = oracle.ref_optimize_frames([d.data_ptr() for d in depth], [n.data_ptr() for n in normal], w.H, w.W, w.K, w.corr, w.poses_init)
-        out_b = o.optimizeWindows([SolveWindow(w.corr, w.H, w.W, depth, normal, w.poses_init, w.K, dense_pairs=pairs)])[0]
-        r, t = synth.pose_errors(out_b, ref_b)
-        print(f"N=30 vs live reference kernels: rot {r:.2e} rad trans {t:.2e} m ({len(pairs)} dense pairs)")
-        assert r <= 3e-4 and t <= 2e-4, (r, t)
+    g = _ref_runs()
+    assert np.allclose(w.poses_init, g["n30_init"], rtol=0, atol=1e-6)
+    ref_b, pairs = g["n30_poses"], g["n30_pairs"]
+    out_b = o.optimizeWindows([SolveWindow(w.corr, w.H, w.W, depth, normal, w.poses_init, w.K, dense_pairs=pairs)])[0]
+    r, t = synth.pose_errors(out_b, ref_b)
+    print(f"N=30 vs the reference's kernels: rot {r:.2e} rad trans {t:.2e} m ({len(pairs)} dense pairs)")
+    assert r <= 3e-4 and t <= 2e-4, (r, t)
     o.close()
 
 
 def test_parity_sweep_against_live_reference(cuda_device):
     """How often does a window fall outside north_star's 1e-4 rad / 1e-4 m against the reference's OWN kernels?  200 seeded windows
-    (3-8 frames, 640x480), each solved by the reference (oracle/_ref, live) and by the library with the reference's pair directions.
-    The hard dense gates amplify rounding-level differences on some windows (test_gate_sensitive_window); for every window beyond
-    the tolerance the reference is run a second time: its own float atomics make it differ from ITSELF, and that run-to-run
-    difference is the yardstick the excess is held against."""
+    (3-8 frames, 640x480), each solved by the reference (its poses and pair directions recorded on a B200) and by the library with the
+    reference's pair directions.  The hard dense gates amplify rounding-level differences on some windows (test_gate_sensitive_window);
+    the reference was run twice on every window: its own float atomics make it differ from ITSELF, and that run-to-run difference is
+    the yardstick the excess is held against."""
     from bundletrack_b200.optimizer import OptimizerGpu, SolveWindow
-    if not os.path.exists(os.path.join(os.path.dirname(oracle.__file__), "_ref", "libbt_ref.so")):
-        pytest.skip("oracle/_ref not built")
     import torch
+    g = _ref_runs()
     o = OptimizerGpu(None, max_windows=1, max_frames=8, max_corr=2000)
     errs, beyond, self_jitter = [], [], []
     n_seeds = 200
+    f0 = p0 = 0
     for seed in range(n_seeds):
         N = 3 + seed % 6
         w = synth.make_window(5000 + seed, n_frames=N, n_corr=200 * N)
+        assert abs(w.poses_init.astype(np.float64).sum() - g["sweep_init_sum"][seed]) <= 1e-5, seed
+        ref = g["sweep_poses"][f0:f0 + N]
+        pairs = g["sweep_pairs"][p0:p0 + g["sweep_n_pairs"][seed]].astype(np.uint32)
+        f0 += N; p0 += len(pairs)
         depth = [torch.from_numpy(w.depth[k]).to(cuda_device) for k in range(N)]
         normal = [torch.from_numpy(w.normal[k]).to(cuda_device) for k in range(N)]
-        dp, nq = [d.data_ptr() for d in depth], [n.data_ptr() for n in normal]
-        ref, pairs, _, _ = oracle.ref_optimize_frames(dp, nq, w.H, w.W, w.K, w.corr, w.poses_init)
         out = o.optimizeWindows([SolveWindow(w.corr, w.H, w.W, depth, normal, w.poses_init, w.K, dense_pairs=pairs)])[0]
         e = max(synth.pose_errors(out, ref))
         errs.append(e)
         if e > TOL:
-            ref2 = oracle.ref_optimize_frames(dp, nq, w.H, w.W, w.K, w.corr, w.poses_init)[0]
             a = oracle.solve_window(w.depth, w.normal, w.K, w.corr, w.poses_init, pairs=pairs)
-            beyond.append((seed, N, e)); self_jitter.append((max(synth.pose_errors(ref2, ref)), max(synth.pose_errors(a, ref))))
+            beyond.append((seed, N, e)); self_jitter.append((float(g["sweep_jitter"][seed]), max(synth.pose_errors(a, ref))))
     errs = np.asarray(errs)
-    print(f"parity sweep vs live reference kernels: {n_seeds} windows; median {np.median(errs):.2e}, p90 {np.percentile(errs, 90):.2e}, p99 {np.percentile(errs, 99):.2e}, max {errs.max():.2e}; "
+    print(f"parity sweep vs the reference's kernels: {n_seeds} windows; median {np.median(errs):.2e}, p90 {np.percentile(errs, 90):.2e}, p99 {np.percentile(errs, 99):.2e}, max {errs.max():.2e}; "
           f"{len(beyond)} beyond 1e-4: {[(s_, n_, float(f'{e_:.1e}')) for s_, n_, e_ in beyond]}; on those, reference run-to-run / oracle A vs reference: {[(float(f'{x:.1e}'), float(f'{y:.1e}')) for x, y in self_jitter]}")
     assert np.median(errs) <= 2e-5 and np.percentile(errs, 90) <= TOL, (np.median(errs), np.percentile(errs, 90))
     o.close()
